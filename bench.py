@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path (one process per GPU)
     python bench.py --impl reference --gpus N --steps K ...  # reference algorithm on the host CPU cores
+    python bench.py ... --dump-outputs DIR                   # + the last timed step's outputs as DIR/*.npy
 
 Workload (BASELINE.json configs[1] / SURVEY.md §8d): bccwj-suw-shaped synthetic model (W=3/3, 300 000 char
 1-3-gram patterns, 258 type n-grams, no dictionary, no tags) over synthetic 40-char Japanese sentences,
@@ -16,11 +17,14 @@ from __future__ import annotations
 
 import argparse
 import ctypes as C
+import functools
+import hashlib
 import json
 import os
 import statistics
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -31,19 +35,24 @@ for p in (ROOT, os.path.join(ROOT, "tests")):
 
 import numpy as np  # noqa: E402
 
-CACHE = os.path.join(ROOT, "bench_cache")
+# Generated models are cached outside the source tree (which may be read-only), per user.  The file name carries a hash
+# of the generator's source, so two builds of the project never read each other's model.
+CACHE = os.path.join(tempfile.gettempdir(), f"vaporetto_b200_bench_cache_{os.getuid()}")
 METRIC = "UTF-8 MB/s segmented (bit-exact i32 scores)"
+DUMP_BYTES = 64_000_000
+DUMP_SEED = 0x5EED0D0
 
 
 def log(*a):
     print(*a, file=sys.stderr, flush=True)
 
 
+@functools.lru_cache(maxsize=None)
 def get_model(n_patterns: int, sample: int, config: int = 2) -> bytes:
     from vpt_testlib import synth
-    os.makedirs(CACHE, exist_ok=True)
     tag = {2: "bccwj_shaped", 3: "bccwj_tags_shaped", 4: "kytea_shaped"}[config]
-    fn = os.path.join(CACHE, f"{tag}_{n_patterns}_{sample}.bin")
+    src = hashlib.sha256(open(synth.__file__, "rb").read()).hexdigest()[:16]
+    fn = os.path.join(CACHE, f"{tag}_{n_patterns}_{sample}_{src}.bin")
     if os.path.exists(fn):
         return open(fn, "rb").read()
     t = time.time()
@@ -51,12 +60,33 @@ def get_model(n_patterns: int, sample: int, config: int = 2) -> bytes:
                                      dict_words=500_000 if config == 4 else 0, tag_models=20_000 if config == 3 else 0)
     log(f"[bench] generated model ({len(m)} bytes) in {time.time() - t:.1f}s")
     try:
+        os.makedirs(CACHE, exist_ok=True)
         with open(fn + ".tmp", "wb") as f:
             f.write(m)
         os.replace(fn + ".tmp", fn)
     except OSError:
         pass
     return m
+
+
+def dump_outputs(out_dir: str, arrays, budget: int = DUMP_BYTES, prefix: str = "") -> None:
+    """Writes the outputs of one step as <out_dir>/<prefix><name>.npy in float64, exact for every i32 / u32 value and for
+    offsets below 2^53.  `arrays`: {name: (tensor, numpy dtype its elements are read as)}.  An array larger than its share
+    of `budget` bytes is written as its values at a fixed, seeded sample of positions (ascending), the positions beside it
+    as <name>_index.npy; the same arguments give the same positions, so two builds can be compared output for output."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    share = budget // len(arrays)
+    for name, (t, dtype) in arrays.items():
+        t = t.reshape(-1)
+        n = t.numel()
+        if 8 * n + 128 > share:   # (128: the .npy header)
+            k = (share - 256) // 16
+            idx = np.sort(np.random.default_rng(DUMP_SEED).choice(n, k, replace=False))
+            np.save(os.path.join(out_dir, f"{prefix}{name}_index.npy"), idx.astype(np.float64))
+            t = t[torch.from_numpy(idx).to(t.device)]
+        v = t.cpu().numpy().view(dtype).astype(np.float64)
+        np.save(os.path.join(out_dir, f"{prefix}{name}.npy"), v)
 
 
 def get_text(n_sent: int, rank: int, ragged: bool):
@@ -328,6 +358,10 @@ def main():
                          "emitted), 4 KyTea-shaped (+ 500K-word dictionary)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--e2e-steps", type=int, default=5)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed (scores, boundaries, offsets, status; "
+                         "config 3: also the pattern-id states) as DIR/<name>.npy, float64, at most 64 MB in all "
+                         "(a fixed, seeded sample of each larger array)")
     args = ap.parse_args()
 
     rank = int(os.environ.get("RANK", "0"))
@@ -422,6 +456,15 @@ def main():
     e1.record(stream)
     barrier()
     ms = e0.elapsed_time(e1)
+    if args.dump_outputs:   # before the profiled leg below overwrites the buffers
+        outs = {"scores": (d_scores[:n_bound], np.int32), "boundaries": (d_bounds[:n_bound], np.uint8),
+                "bound_offsets": (d_boff, np.int64), "status": (d_status, np.int32)}
+        if want_states:
+            n_chars = int(d_coff[-1].item())
+            outs.update(char_states=(d_cst[:n_chars], np.uint32), type_states=(d_tst[:n_chars], np.uint32),
+                        char_offsets=(d_coff, np.int64))
+        dump_outputs(args.dump_outputs, outs, DUMP_BYTES // world, f"rank{rank}_" if world > 1 else "")
+        log(f"[bench] rank {rank}: outputs of the last timed step written to {args.dump_outputs}")
     # stage timing of the dominant kernel (CUDA events inside the library, same stream)
     stage = (C.c_float * 3)()
     stage_acc = np.zeros(3)
